@@ -18,6 +18,8 @@ fixed), one NCCL all-gather of the decoded ids per step.  A "step" is one pass o
                  timed on the host cores on ONE full-depth image with a shortened decode (stated in ``sample``); the oracle
                  port (``kind: "port"``) only if that copy is absent.
 ``--impl reference`` times that CPU arm alone: one full-depth image per step, all decode tokens, every host thread.
+``--dump-outputs DIR`` writes what the last timed step (of rank 0) returned as DIR/<name>.npy (dump_outputs); weights and inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 Workloads (``--workload``): c3 (default, the headline configuration), c4 (COCO shape: 640 px -> 46x46 grid, 100 boxes,
 16 images / GPU), c5 (counting: 1344 px, 300 boxes, 128 tokens, 8 images / GPU), c2 (HFRE-only: towers + region tokens of
@@ -185,6 +187,33 @@ def hfre_algorithmic_bytes(HF, cfg, host, size):
     return tot
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(res: dict, out_dir: str) -> None:
+    """Write the arrays one step returned as <out_dir>/<name>.npy: integers (token ids, lengths) as float64, which holds them
+    exactly, floating-point values as float32.  An array larger than its share of DUMP_BYTES keeps a seeded sample of its rows,
+    the same rows on every run, whose indices go to <name>_rows.npy."""
+    arrays = {}
+    for k, v in res.items():
+        if v is None:
+            continue
+        if torch.is_tensor(v):
+            v = v.detach().cpu()
+            v = v.float() if v.is_floating_point() else v
+        a = np.asarray(v)
+        arrays[k] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(len(arrays), 1) - 1024          # room for the .npy headers
+    for k, a in arrays.items():
+        if a.nbytes > share:
+            row_bytes = a.nbytes // a.shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // (row_bytes + 8), replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{k}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def load_traffic(workload: str, per_gpu_batch: int):
     """DRAM bytes per launch of the roofline kernels from the committed ncu capture of this round (profiles/): the bench
     cannot run under ncu, so `traffic` is read from the capture of the same command -- one C3 step at 32 images per GPU
@@ -213,7 +242,13 @@ def main():
     ap.add_argument("--cpu-tokens", type=int, default=64, help="decode steps the in-run cpu_baseline executes (rest at the measured per-token time)")
     ap.add_argument("--profile-run", action="store_true", help="warm-up exactly as given, one timed pass, nothing else (for ncu)")
     ap.add_argument("--small", action="store_true", help="tiny architecture (plumbing check only; NOT a valid bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path (--impl fo1)")
     wl = WORKLOADS[args.workload]
     for k in ("batch", "size", "boxes", "tokens"):
         if getattr(args, k) is None:
@@ -249,9 +284,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        # bounded: a step is ONE full-depth image (~45 s on the 16 cores a box grants); one untimed warm-up step (if any was asked for)
-        # and at most two timed ones, so that any --steps K --warmup W ends within a few minutes of host time
-        steps = max(1, min(args.steps, 2))
+        # a step is ONE full-depth image (~45 s on 16 host cores); the untimed warm-up is bounded to one step (if any was asked for)
+        steps = args.steps
         ips, kind, cores, note, detail = reference_arm(args, cfg, steps, min(args.cpu_tokens, max(T, 1)), warm=min(args.warmup, 1))
         value = ips
         if hfre_only:                                # the HFRE stage alone, same unit as the GPU arm
@@ -312,27 +346,30 @@ def main():
         return res
 
     def timed(fn, steps):
+        """-> (ms of the steps, what the last step returned)"""
         if dist is not None:
             dist.barrier()
         torch.cuda.synchronize()
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            res = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if dist is not None:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), res
 
     L = fo1_b200.lib()
     if args.profile_run:
         for _ in range(args.warmup):
             step(resident)
-        ms = timed(lambda: step(resident), args.steps)
+        ms, res = timed(lambda: step(resident), args.steps)
         if rank == 0:
+            if args.dump_outputs:
+                dump_outputs(res, args.dump_outputs)
             print(json.dumps({"profile_run": True, "ms_per_step": ms / args.steps, "launches": int(L.fo1_launch_count())}), file=out, flush=True)
         return
     for _ in range(max(args.warmup, 3)):
@@ -340,12 +377,15 @@ def main():
     torch.cuda.synchronize()
     L.fo1_launch_count_reset()
     with ClockSampler(local) as cs:
-        ms = timed(lambda: step(resident), args.steps)
+        ms, res = timed(lambda: step(resident), args.steps)
     launches = int(L.fo1_launch_count())
     clocks = cs.summary()
     ips = G * args.steps / (ms / 1000.0)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
+    del res
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     ips_e2e = G * args.steps / (ms_e2e / 1000.0)
     h2d = sum(s.image_u8.numel() + s.boxes.numel() * 4 for s in host_u8)
     d2h = host_regions.numel() * 2 if hfre_only else B * Tc * 4

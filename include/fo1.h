@@ -87,7 +87,8 @@ typedef struct {
   int32_t out_dim;          /* D = mm_region_hidden_size (5888 variant B, 8960 variant A) */
   int32_t roi_size;         /* 7 (omchat_arch.py:18) */
   int32_t apply_pos_embed;  /* mm_apply_position_embedding, bbox_based */
-  int32_t algo;             /* 0 = auto, 1 = per-box gather, 2 = map sweep (SIMT), 3 = map sweep, row sums on mma.sync */
+  int32_t algo;             /* 0 = auto (gather below 8 boxes per image on average, else sweep), 1 = per-box gather,
+                               3 = map sweep, row sums on mma.sync; other values are rejected */
 } fo1_hfre_params;
 
 /* Bytes of device workspace fo1_hfre_forward needs for these images (host-side arithmetic only). */

@@ -1,5 +1,5 @@
-"""Decode-loop probe: per-step decode time at B=32, L=1195 (prefill-only vs 64-token run), with and without the CUDA
-graph; under ncu (FO1_NO_GRAPH=1, few steps) it yields the exact per-kernel durations of one decode step."""
+"""Decode-loop probe: per-step decode time at B=32, L=1195 (prefill-only vs 64-token run); under ncu (PROBE_NCU=1, few steps)
+it yields the exact per-kernel durations of one decode step."""
 import json
 import os
 import sys
@@ -48,5 +48,5 @@ elif os.environ.get("PROBE_NCU"):
 else:
     run(4); run(4)
     p = min(run(1) for _ in range(3)); f = min(run(T) for _ in range(3))
-    print(json.dumps({"B": B, "L": L, "T": T, "graph": os.environ.get("FO1_NO_GRAPH") is None, "prefill_ms": p, "full_ms": f,
+    print(json.dumps({"B": B, "L": L, "T": T, "prefill_ms": p, "full_ms": f,
                       "decode_ms_per_step": (f - p) / (T - 1)}))

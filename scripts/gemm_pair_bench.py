@@ -1,4 +1,4 @@
-"""python scripts/gemm_pair_bench.py: CTA-pair GEMM vs the single-CTA kernel (FO1_GEMM_NO_PAIR=1) at the step's big shapes, warm clocks."""
+"""python scripts/gemm_pair_bench.py: CTA-pair GEMM vs the single-CTA kernel (pinned tile_n=256) at the step's big shapes, warm clocks."""
 import os, sys, time
 import torch
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -19,12 +19,11 @@ for M, N, K, gated in shapes:
     res = {}
     for rep in range(2):
         for tag in ("pair", "single"):
-            if tag == "single": os.environ["FO1_GEMM_NO_PAIR"] = "1"
-            else: os.environ.pop("FO1_GEMM_NO_PAIR", None)
-            for _ in range(3): ops.gemm(a, w, gated=gated, act="silu" if gated else None, out=out)
+            tn = 256 if tag == "single" else 0
+            for _ in range(3): ops.gemm(a, w, gated=gated, act="silu" if gated else None, out=out, tile_n=tn)
             e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
             e0.record()
-            for _ in range(10): ops.gemm(a, w, gated=gated, act="silu" if gated else None, out=out)
+            for _ in range(10): ops.gemm(a, w, gated=gated, act="silu" if gated else None, out=out, tile_n=tn)
             e1.record(); torch.cuda.synchronize()
             ms = e0.elapsed_time(e1) / 10
             res[tag] = min(res.get(tag, 1e9), ms)

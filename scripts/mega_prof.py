@@ -1,7 +1,6 @@
 """FO1_MEGA_PROF=1 python scripts/mega_prof.py [B] [L]: one generate() of the LLM alone at the 3B widths, prints the per-phase profile
 of the persistent decode kernel (stderr) and the decode step time with / without it."""
 import os, sys, time
-os.environ.setdefault("FO1_MEGA_MAX_B", "32")
 import torch
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO)

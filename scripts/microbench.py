@@ -103,7 +103,7 @@ def bench_hfre(results, B=8, S=896, N=100, algo=0):
     L.fo1_profile_enable(0)
     prof = json.loads(buf.value.decode())
     kern = {k: round(v["ms"] / v["launches"], 4) for k, v in prof.items()}
-    main = kern.get("hfre_sweep_mma") or kern.get("hfre_sweep") or kern.get("hfre_gather")
+    main = kern.get("hfre_sweep_mma") or kern.get("hfre_gather")
     r = {"kind": "hfre", "algo": algo, "B": B, "S": S, "N": N, "ms": med, "kernel_ms": kern,
          "kernel_unique_GBs": tot_unique / main / 1e6, "kernel_frac_of_measured_hbm": tot_unique / main / 1e6 / PEAKS["hbm_gbs"], "ms_best": best, "unique_MB": tot_unique / 1e6, "gather_MB": tot_gather / 1e6,
          "unique_GBs": tot_unique / med / 1e6, "gather_GBs": tot_gather / med / 1e6,
@@ -134,9 +134,9 @@ if __name__ == "__main__":
     res = []
     print("device", torch.cuda.get_device_name(0), "cpus", os.cpu_count(), flush=True)
     if "hfre" in which:
-        for algo in (1, 2, 3):
+        for algo in (1, 3):
             bench_hfre(res, algo=algo)
-        for algo in (1, 2, 3):
+        for algo in (1, 3):
             bench_hfre(res, B=8, S=896, N=32, algo=algo)     # COCO-like box count (mean 31.5)
     if "gemm" in which:
         bench_gemm(res)

@@ -28,7 +28,7 @@ if "skinny" in which:
         ops.gemm(a, w, act="silu", gated=True)
 if "hfre" in which:
     aux_all, pyr_all, ba, bv, grids = MB.make_hfre_inputs(8, 896, 100)
-    for algo in [int(a) for a in os.environ.get("NCU_HFRE_ALGOS", "1,2,3").split(",")]:
+    for algo in [int(a) for a in os.environ.get("NCU_HFRE_ALGOS", "1,3").split(",")]:
         cfg = H.HfreConfig(region_dim=5888, vt_mode="fpn", algo=algo)
         for _ in range(2):
             H.hfre_forward(aux_all, pyr_all, ba, bv, cfg, grids)

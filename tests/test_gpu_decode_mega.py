@@ -12,13 +12,6 @@ import torch
 pytestmark = pytest.mark.gpu
 
 
-
-@pytest.fixture(autouse=True)
-def _mega_up_to_32(monkeypatch):
-    """The default threshold is 16 sequences (llm.cu); these tests cover both row-tile variants of the kernel."""
-    monkeypatch.setenv("FO1_MEGA_MAX_B", "32")
-
-
 def _engine(layers=2, vocab=32000):
     from importlib import import_module
     import fo1_b200  # noqa: F401

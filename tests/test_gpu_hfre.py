@@ -16,7 +16,7 @@ def _nerr(got, ref):
     return float((got - ref).abs().max() / ref.abs().max())
 
 
-@pytest.mark.parametrize("algo", [1, 2, 3])
+@pytest.mark.parametrize("algo", [1, 3])
 @pytest.mark.parametrize("tag", ["small", "rect"])
 def test_hfre_matches_reference_goldens(golden_dir, tag, algo):
     import fo1_b200  # noqa: F401
@@ -39,7 +39,7 @@ def test_hfre_matches_reference_goldens(golden_dir, tag, algo):
     np.testing.assert_allclose(out_a.cpu().numpy(), z["out_concat"], rtol=1e-3, atol=2e-4)
 
 
-@pytest.mark.parametrize("algo", [1, 2, 3])
+@pytest.mark.parametrize("algo", [1, 3])
 @pytest.mark.parametrize("S,N", [(448, 37), (896, 100)])
 def test_hfre_matches_oracle_full_shapes(S, N, algo):
     """DaViT-large / SimpleFPN shaped maps at real resolution, batch of 2 images, ragged box counts."""
@@ -87,6 +87,8 @@ def test_hfre_empty_and_errors():
     one = torch.tensor([[0.0, 0.0, 4.0, 4.0]], device="cuda")
     with pytest.raises(L.Fo1Error):
         H.hfre_forward([bad], [pyr], [one], [one], H.HfreConfig(region_dim=128), [(2, 2)])
+    with pytest.raises(L.Fo1Error):   # algo: 0 auto, 1 gather, 3 sweep
+        H.hfre_forward([aux], [pyr], [one], [one], H.HfreConfig(region_dim=128, algo=2), [(2, 2)])
 
 
 def test_hfre_packed_batch_is_the_same_operator():

@@ -454,9 +454,9 @@ static int launch_attn_tc(const AttnArgs& a, const int2* rowseg, cudaStream_t s)
   ProfScope prof(CAUSAL ? "attn_causal" : "attn", a.flops, 0.0, s);
   // persistent for the non-causal shapes (equal-cost items: ViT / DaViT windows 0.40 -> 0.33 ms, 0.78 -> 0.66 ms per layer at 32 images): two
   // CTAs per SM walk the item list.  Causal prompts have items of very different cost; the static round robin lost 19 % against the
-  // hardware block scheduler there, so they keep one CTA per item (the same kernel with a one-item list).  FO1_ATTN_ONE_ITEM: A/B knob.
+  // hardware block scheduler there, so they keep one CTA per item (the same kernel with a one-item list).
   const long long resident = 2LL * device_sm_count();
-  const unsigned grid = (unsigned)((CAUSAL || getenv("FO1_ATTN_ONE_ITEM") != nullptr || blocks < resident) ? blocks : resident);
+  const unsigned grid = (unsigned)((CAUSAL || blocks < resident) ? blocks : resident);
   attn_tc_kernel<HD, CAUSAL><<<grid, kAtThreads, Cfg::kSmemBytes, s>>>(tmQ, tmK, tmV, g);
   FO1_LAUNCH_CHECK();
   return FO1_OK;

@@ -887,6 +887,26 @@ static int splitk_scratch(cudaStream_t stream, size_t need_bytes, int need_count
 
 struct ConvInfo { int B, H, W, C, Wt; };   // implicit 3x3 conv: d->A is the NHWC map, d->M = B*H*W, d->K = 9*C
 
+// the GemmArgs fields both kernels take from the descriptor and the conv geometry; tiling, ring stages and split-K are
+// left zero for the launcher to plan
+static GemmArgs gemm_args(const fo1_gemm_desc* d, const ConvInfo* conv) {
+  GemmArgs g;
+  memset(&g, 0, sizeof(g));
+  g.M = d->M; g.N = d->N; g.K = d->K;
+  g.D = d->D; g.ldd = d->ldd; g.d_dtype = d->d_dtype;
+  g.bias = d->bias; g.bias_dtype = d->bias_dtype;
+  g.act = d->act;
+  g.residual = static_cast<const __nv_bfloat16*>(d->residual); g.ldr = d->ldr;
+  g.gated = d->gated;
+  g.conv_cpb = conv ? conv->C / BK : 0; g.conv_H = conv ? conv->H : 0; g.conv_W = conv ? conv->W : 0; g.conv_Wt = conv ? conv->Wt : 0;
+  g.tiles_m = ceil_div(d->M, BM);
+  const int esz = d->d_dtype == FO1_BF16 ? 2 : 4;
+  const bool d_ok = (reinterpret_cast<uintptr_t>(d->D) & 15) == 0 && (d->ldd * esz) % 16 == 0;
+  const bool r_ok = d->residual == nullptr || ((reinterpret_cast<uintptr_t>(d->residual) & 15) == 0 && (d->ldr * 2) % 16 == 0);
+  g.coalesce = (d_ok && r_ok) ? 1 : 0;
+  return g;
+}
+
 template <int BN>
 static int launch_gemm(const fo1_gemm_desc* d, cudaStream_t stream, int ksplit = 1, const ConvInfo* conv = nullptr) {
   using Cfg = GemmCfg<BN>;
@@ -905,15 +925,7 @@ static int launch_gemm(const fo1_gemm_desc* d, cudaStream_t stream, int ksplit =
     FO1_TRY(make_tmap_2d_bf16(&tmA, d->A, (uint64_t)d->K, (uint64_t)d->M, (uint64_t)d->lda, BK, a_rows));
   }
   FO1_TRY(make_tmap_2d_bf16(&tmW, d->W, (uint64_t)d->K, (uint64_t)d->N, (uint64_t)d->ldw, BK, BN));
-  GemmArgs g;
-  g.M = d->M; g.N = d->N; g.K = d->K;
-  g.D = d->D; g.ldd = d->ldd; g.d_dtype = d->d_dtype;
-  g.bias = d->bias; g.bias_dtype = d->bias_dtype;
-  g.act = d->act;
-  g.residual = static_cast<const __nv_bfloat16*>(d->residual); g.ldr = d->ldr;
-  g.gated = d->gated;
-  g.conv_cpb = conv ? conv->C / BK : 0; g.conv_H = conv ? conv->H : 0; g.conv_W = conv ? conv->W : 0; g.conv_Wt = conv ? conv->Wt : 0;
-  g.tiles_m = ceil_div(d->M, BM);
+  GemmArgs g = gemm_args(d, conv);
   g.tiles_n = ceil_div(d->N, BN);
   g.stage_tx = (a_rows + BN) * BK * 2;
   // the UMMA reads all 128 A rows of a stage: keep the full 16 KB slot unless only the live rows are loaded AND the
@@ -927,17 +939,9 @@ static int launch_gemm(const fo1_gemm_desc* d, cudaStream_t stream, int ksplit =
     while (st > 2 && st * (g.a_stage_bytes + g.b_stage_bytes) + (BM * BK * 2 - g.a_stage_bytes) > budget) --st;
     g.stages = st < kMaxStages ? st : kMaxStages;
   }
-  {
-    const int esz = d->d_dtype == FO1_BF16 ? 2 : 4;
-    const bool d_ok = (reinterpret_cast<uintptr_t>(d->D) & 15) == 0 && (d->ldd * esz) % 16 == 0;
-    const bool r_ok = d->residual == nullptr || ((reinterpret_cast<uintptr_t>(d->residual) & 15) == 0 && (d->ldr * 2) % 16 == 0);
-    static const bool direct_store = getenv("FO1_GEMM_DIRECT_STORE") != nullptr;   // A/B knob: per-row stores instead of the smem-staged lines
-    g.coalesce = (d_ok && r_ok && !direct_store) ? 1 : 0;
-  }
   const int num_kb = ceil_div(d->K, BK);
   g.kb_per_split = ceil_div(num_kb, ksplit);
   g.ksplit = ceil_div(num_kb, g.kb_per_split);   // every split owns at least one k-block
-  g.ws = nullptr; g.counters = nullptr;
   if (g.ksplit > 1) {
     SplitKScratch* sc = nullptr;
     FO1_TRY(splitk_scratch(stream, (size_t)g.tiles_m * g.tiles_n * g.ksplit * BM * BN * sizeof(float), g.tiles_m * g.tiles_n, &sc));
@@ -968,26 +972,10 @@ static int launch_gemm_pair(const fo1_gemm_desc* d, cudaStream_t stream, const C
     FO1_TRY(make_tmap_2d_bf16(&tmA, d->A, (uint64_t)d->K, (uint64_t)d->M, (uint64_t)d->lda, BK, BM));
   }
   FO1_TRY(make_tmap_2d_bf16(&tmW, d->W, (uint64_t)d->K, (uint64_t)d->N, (uint64_t)d->ldw, BK, kPairBN / 2));
-  GemmArgs g;
-  memset(&g, 0, sizeof(g));
-  g.M = d->M; g.N = d->N; g.K = d->K;
-  g.D = d->D; g.ldd = d->ldd; g.d_dtype = d->d_dtype;
-  g.bias = d->bias; g.bias_dtype = d->bias_dtype;
-  g.act = d->act;
-  g.residual = static_cast<const __nv_bfloat16*>(d->residual); g.ldr = d->ldr;
-  g.gated = d->gated;
-  g.conv_cpb = conv ? conv->C / BK : 0; g.conv_H = conv ? conv->H : 0; g.conv_W = conv ? conv->W : 0; g.conv_Wt = conv ? conv->Wt : 0;
-  g.tiles_m = ceil_div(d->M, BM);
+  GemmArgs g = gemm_args(d, conv);
   g.tiles_n = ceil_div(d->N, kPairBN);
   g.ksplit = 1; g.kb_per_split = ceil_div(d->K, BK);
   g.stages = kPairStages;
-  {
-    const int esz = d->d_dtype == FO1_BF16 ? 2 : 4;
-    const bool d_ok = (reinterpret_cast<uintptr_t>(d->D) & 15) == 0 && (d->ldd * esz) % 16 == 0;
-    const bool r_ok = d->residual == nullptr || ((reinterpret_cast<uintptr_t>(d->residual) & 15) == 0 && (d->ldr * 2) % 16 == 0);
-    static const bool direct_store = getenv("FO1_GEMM_DIRECT_STORE") != nullptr;
-    g.coalesce = (d_ok && r_ok && !direct_store) ? 1 : 0;
-  }
   const int work = ((g.tiles_m + 1) / 2) * g.tiles_n;
   const int clusters = std::min(work, device_sm_count() / 2);
   char tag[96] = "gemm";
@@ -998,9 +986,8 @@ static int launch_gemm_pair(const fo1_gemm_desc* d, cudaStream_t stream, const C
   FO1_LAUNCH_CHECK();
   return FO1_OK;
 }
-// one wave of tile pairs at least, whole 128-row A boxes, and not switched off (FO1_GEMM_NO_PAIR: the A/B knob of the parity test)
+// one wave of tile pairs at least, and whole 128-row A boxes
 static bool use_pair_kernel(int M, int N) {
-  if (getenv("FO1_GEMM_NO_PAIR") != nullptr) return false;
   const long long work = (long long)ceil_div(ceil_div(M, BM), 2) * ceil_div(N, kPairBN);
   return M >= BM && N >= kPairBN && work >= device_sm_count() / 2;
 }

@@ -11,12 +11,10 @@
 // because the up-sampling is linear and separable too, U[c] = Mh L[c] Mw^T, the whole thing is
 //        out[c] = (Mh^T a)^T L[c] (Mw^T b)
 // over the NATIVE-resolution bf16 level L (channels-last).  hfre_axis_weights_kernel builds the two weight vectors
-// per (box, level, axis) with torchvision's exact per-sample rules.  Three interchangeable reductions follow
-// (fo1_hfre_params.algo): the per-box gather (coalesced 16-byte channel vectors, fp32 FMA), the SIMT map sweep (every
-// cell read once, FMA per covering box) and -- the default above a handful of boxes -- the map sweep whose row sums
-// run as mma.sync m16n8k16 tiles (boxes x cells, column weights split hi + lo in bf16): the bytes are still read
-// exactly once with coalesced accesses, the legacy tensor path only replaces the FMA issue slots that capped the SIMT
-// sweep at 10 % of the HBM roofline (DESIGN.md section 4).
+// per (box, level, axis) with torchvision's exact per-sample rules.  Two interchangeable reductions follow
+// (fo1_hfre_params.algo): the per-box gather (coalesced 16-byte channel vectors, fp32 FMA), which re-reads a cell once
+// per covering box, and -- the default above a handful of boxes -- the map sweep, which reads every cell once and runs
+// its row sums as mma.sync m16n8k16 tiles (boxes x cells, column weights split hi + lo in bf16; DESIGN.md section 4).
 #include "common.cuh"
 
 namespace fo1 {
@@ -24,11 +22,10 @@ namespace fo1 {
 constexpr int kMaxBatch = 32;          // images per launch: the batch descriptor travels as a kernel parameter (< 32 KB)
 constexpr int kGatherThreads = 256;
 constexpr int kChunk = 256;            // channels per gather block: 32 lanes x 8 bf16 (16 B) each
-constexpr int kRegion = 32;            // sweep: a CTA owns a kRegion x kRegion block of cells of one level
-constexpr int kSweepCh = 256;          // sweep: channels per CTA (4 warps x 32 lanes x 2 channels)
-constexpr int kSlots = 32;             // sweep: boxes accumulated concurrently per pass over the region
+constexpr int kRegion = 32;            // sweep: region width in cells
+constexpr int kSweepCh = 256;          // sweep: channels per CTA (4 warps x 64 channels)
 constexpr int kSweepThreads = 128;
-constexpr int kMmaRows = 8;            // tensor sweep: region = kMmaRows x kRegion cells, one 16-box m-tile per pass
+constexpr int kMmaRows = 8;            // sweep: region = kMmaRows x kRegion cells, one 16-box m-tile per pass
 constexpr int kMmaSlots = 16;
 
 struct LevelDev {
@@ -51,7 +48,7 @@ struct ImageDev {
                      // not depend on the order in which the region CTAs arrive (bit-reproducible, unlike fp32 atomics)
   long long ws_ofs;  // float offset of this image's workspace slice
   long long ls_ofs;  // int offset of this image's region-list slice (after all weight records)
-  int lstride;       // ints per region list: 1 count + n_boxes ids, rounded up to 4
+  int lstride;       // ints per region list: 4 header words (word 0 = count) + one kRecWords record per box
   int n_items;       // sweep work items: sum over levels of regions * ceil(C / kSweepCh)
   float pos_w, pos_h;
   int pos_box_set;
@@ -62,7 +59,6 @@ struct ImageDev {
 struct BatchDev {
   ImageDev img[kMaxBatch];
   int n_images;
-  int rrows;     // region height in cells used by the region lists / sweep of this launch (kRegion or kMmaRows)
   int out_dim;
   int roi;
   int pos;
@@ -303,64 +299,10 @@ __global__ void __launch_bounds__(kGatherThreads) hfre_gather_kernel(const Batch
   }
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Kernel 3' (algo 2, map sweep).  The per-box gather above re-reads every cell once per covering box
-// (~8x the unique bytes at 100 boxes/image, L2-bound).  The sweep inverts the loops: a CTA owns a
-// 32x32-cell region x 256 channels of one level, reads each cell ONCE, and for every box whose
-// support meets the region accumulates a^T L b for its part, box accumulators living in shared
-// memory (lane-owned columns: no intra-CTA atomics); one fp32 red.global.add per (region, box,
-// channel) at the end.  Per cell and covering box the work is 2 FMA per bf16 pair -- the SIMT FMA
-// rate, not HBM, is then the co-limiter (DESIGN.md section 4).
-// ------------------------------------------------------------------------------------------------
-// packed fp32x2 helpers: one FFMA2 does the two channels a lane owns (sm_100 `fma.rn.f32x2`; a {w, w} pair becomes
-// the instruction's scalar-broadcast operand)
-__device__ __forceinline__ unsigned long long f2_pack(float lo, float hi) {
-  unsigned long long r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ unsigned long long f2_fma(unsigned long long a, unsigned long long b, unsigned long long c) {
-  unsigned long long d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
-}
-__device__ __forceinline__ float2 f2_unpack(unsigned long long v) {
-  float2 r;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(v));
-  return r;
-}
-
-__global__ void __launch_bounds__(32) hfre_region_lists_kernel(const BatchDev B, const float* __restrict__ ws, int* __restrict__ lists) {
-  const ImageDev& im = B.img[blockIdx.z];
-  const int lvl = blockIdx.y;
-  if (lvl >= im.n_levels) return;
-  const LevelDev& L = im.lv[lvl];
-  const int reg = blockIdx.x;
-  if (reg >= L.rh * L.rw) return;
-  const int ry = reg / L.rw, rx = reg % L.rw;
-  const int row0 = ry * B.rrows, row1 = min(row0 + B.rrows, L.H) - 1;
-  const int col0 = rx * kRegion, col1 = min(col0 + kRegion, L.W) - 1;
-  int* out = lists + im.ls_ofs + L.lofs + (long long)reg * im.lstride;
-  int count = 0;
-  for (int b0 = 0; b0 < im.n_boxes; b0 += 32) {
-    const int b = b0 + threadIdx.x;
-    bool hit = false;
-    if (b < im.n_boxes) {
-      const int* hdr = reinterpret_cast<const int*>(ws + im.ws_ofs + L.wofs + (long long)b * L.wstride);
-      const int r0 = hdr[0], r1 = hdr[0] + hdr[1] - 1, c0 = hdr[2], c1 = hdr[2] + hdr[3] - 1;
-      hit = r0 <= row1 && r1 >= row0 && c0 <= col1 && c1 >= col0;
-    }
-    const unsigned m = __ballot_sync(0xffffffffu, hit);
-    if (hit) out[1 + count + __popc(m & ((1u << threadIdx.x) - 1u))] = b;
-    count += __popc(m);
-  }
-  if (threadIdx.x == 0) out[0] = count;
-}
-
-// Tensor sweep variant of the region lists: besides the ids, every listed box gets its weights over the region's rows
-// and columns as one contiguous 48-word record (word 0 = box id, words 4..4+kMmaRows-1 = a_y, words 12..43 = b_x), so a
-// sweep pass stages its 16 boxes with ONE round of coalesced loads instead of the id -> header -> weights chain.
+// Region lists of the sweep below: per region, the boxes whose support meets it.  Every listed box gets its weights over
+// the region's rows and columns as one contiguous 48-word record (word 0 = box id, words 4..4+kMmaRows-1 = a_y, words
+// 12..43 = b_x), so a sweep pass stages its 16 boxes with ONE round of coalesced loads instead of the id -> header ->
+// weights chain.
 constexpr int kRecWords = 48;
 static_assert(kMmaRows <= 8 && kRegion == 32, "record layout: words 4..11 = a_y, words 12..43 = b_x");
 __global__ void __launch_bounds__(128) hfre_region_records_kernel(const BatchDev B, const float* __restrict__ ws, int* __restrict__ lists) {
@@ -406,112 +348,12 @@ __global__ void __launch_bounds__(128) hfre_region_records_kernel(const BatchDev
   }
 }
 
-__global__ void __launch_bounds__(kSweepThreads) hfre_sweep_kernel(const BatchDev B, const float* __restrict__ ws, const int* __restrict__ lists) {
-  const ImageDev& im = B.img[blockIdx.z];
-  if ((int)blockIdx.x >= im.n_items) return;
-  int lvl = 0, item = blockIdx.x;
-  for (; lvl < im.n_levels; ++lvl) {
-    const int n = im.lv[lvl].rh * im.lv[lvl].rw * ((im.lv[lvl].C + kSweepCh - 1) / kSweepCh);
-    if (item < n) break;
-    item -= n;
-  }
-  const LevelDev& L = im.lv[lvl];
-  const int n_reg = L.rh * L.rw;
-  const int cgroup = item / n_reg, reg = item % n_reg;
-  const int* list = lists + im.ls_ofs + L.lofs + (long long)reg * im.lstride;
-  const int n_list = list[0];
-  if (n_list == 0) return;  // no box touches this region: its cells are never read
-  const int ry = reg / L.rw, rx = reg % L.rw;
-  const int row0 = ry * kRegion, col0 = rx * kRegion;
-
-  __shared__ __align__(16) float s_acc[kSlots][kSweepCh];
-  __shared__ __align__(16) float s_wa[kSlots][kRegion];
-  __shared__ __align__(16) float s_wb[kSlots][kRegion];
-  __shared__ int s_box[kSlots];
-  __shared__ int s_rmask[kSlots], s_cmask[kSlots];   // which 8-row / 8-col tile bands carry non-zero weights
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int cbase = cgroup * kSweepCh + warp * 64 + lane * 2;
-  const bool active = cbase < L.C;
-  const long long rowpitch = (long long)L.W * L.C;
-
-  for (int base = 0; base < n_list; base += kSlots) {
-    const int ns = min(kSlots, n_list - base);
-    // ---- stage this pass's boxes: ids, dense weights over the region's rows / cols, band masks ----
-    if (threadIdx.x < kSlots) {
-      s_box[threadIdx.x] = threadIdx.x < ns ? list[1 + base + threadIdx.x] : -1;
-      s_rmask[threadIdx.x] = 0; s_cmask[threadIdx.x] = 0;
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < ns * kRegion * 2; i += kSweepThreads) {
-      const int sl = i / (kRegion * 2), j = i % (kRegion * 2);
-      const int axis = j / kRegion, k = j % kRegion;
-      const float* rec = ws + im.ws_ofs + L.wofs + (long long)s_box[sl] * L.wstride;
-      const int* hdr = reinterpret_cast<const int*>(rec);
-      const int start = hdr[axis * 2], len = hdr[axis * 2 + 1];
-      const int idx = (axis ? col0 : row0) + k - start;
-      const float w = (idx >= 0 && idx < len) ? rec[4 + (axis ? L.H : 0) + idx] : 0.0f;
-      (axis ? s_wb : s_wa)[sl][k] = w;
-      if (w != 0.0f) atomicOr(axis ? &s_cmask[sl] : &s_rmask[sl], 1 << (k >> 3));
-    }
-    for (int i = threadIdx.x; i < ns * kSweepCh; i += kSweepThreads) s_acc[i / kSweepCh][i % kSweepCh] = 0.0f;
-    __syncthreads();
-
-    if (active) {
-      for (int tile = 0; tile < 16; ++tile) {
-        const int ty = tile >> 2, tx = tile & 3;
-        const int r_base = row0 + ty * 8, c_base = col0 + tx * 8;
-        if (r_base >= L.H || c_base >= L.W) continue;
-        bool any = false;
-        for (int sl = 0; sl < ns; ++sl) any |= ((s_rmask[sl] >> ty) & 1) && ((s_cmask[sl] >> tx) & 1);
-        if (!any) continue;  // warp-uniform
-        unsigned long long v2[8][8];   // (channel 0, channel 1) of the 64 cells, packed fp32x2
-        const __nv_bfloat16* p0 = L.data + (long long)r_base * rowpitch + (long long)c_base * L.C + cbase;
-#pragma unroll
-        for (int r = 0; r < 8; ++r) {
-#pragma unroll
-          for (int k = 0; k < 8; ++k) {
-            uint32_t u = 0;
-            if (r_base + r < L.H && c_base + k < L.W) u = __ldg(reinterpret_cast<const uint32_t*>(p0 + (long long)r * rowpitch + (long long)k * L.C));
-            v2[r][k] = f2_pack(bf16_lo(u), bf16_hi(u));
-          }
-        }
-        for (int sl = 0; sl < ns; ++sl) {
-          if (!(((s_rmask[sl] >> ty) & 1) && ((s_cmask[sl] >> tx) & 1))) continue;
-          const float4 b0 = *reinterpret_cast<const float4*>(&s_wb[sl][tx * 8]), b1 = *reinterpret_cast<const float4*>(&s_wb[sl][tx * 8 + 4]);
-          const float4 a0 = *reinterpret_cast<const float4*>(&s_wa[sl][ty * 8]), a1 = *reinterpret_cast<const float4*>(&s_wa[sl][ty * 8 + 4]);
-          const float wb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-          const float wa[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-          unsigned long long a2 = 0ull;
-#pragma unroll
-          for (int r = 0; r < 8; ++r) {
-            unsigned long long t2 = 0ull;
-#pragma unroll
-            for (int k = 0; k < 8; ++k) t2 = f2_fma(f2_pack(wb[k], wb[k]), v2[r][k], t2);
-            a2 = f2_fma(f2_pack(wa[r], wa[r]), t2, a2);
-          }
-          const float2 part = f2_unpack(a2);
-          float2* acc = reinterpret_cast<float2*>(&s_acc[sl][warp * 64 + lane * 2]);  // lane-owned: no atomics
-          float2 cur = *acc;
-          cur.x += part.x; cur.y += part.y;
-          *acc = cur;
-        }
-      }
-    }
-    __syncthreads();
-    // ---- flush: one fp32 reduction per (box, channel) of this region ----
-    for (int i = threadIdx.x; i < ns * kSweepCh; i += kSweepThreads) {
-      const int sl = i / kSweepCh, c = cgroup * kSweepCh + (i % kSweepCh);
-      if (c < L.C) acc_add(im.acc + (long long)s_box[sl] * B.out_dim + L.out_off + c, s_acc[sl][i % kSweepCh]);
-    }
-    __syncthreads();
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
-// Kernel 3'' (algo 3, map sweep on the tensor pipe).  At C2's box density every cell is covered by ~7 boxes, i.e.
-// ~7.5 FLOP per loaded byte: with the bf16 -> fp32 unpacking the SIMT sweep is issue-bound at ~1/8 of the HBM roofline
-// (profiles/: FMA pipe 26 %, 488 M warp instructions for 1.3 GB).  The reduction is a contraction,
+// Kernel 3' (algo 3, map sweep on the tensor pipe).  The per-box gather re-reads every cell once per covering box (~8x
+// the unique bytes at 100 boxes/image, L2-bound); the sweep inverts the loops so that a CTA reads each cell of its region
+// once.  At C2's box density every cell is covered by ~7 boxes, i.e. ~7.5 FLOP per loaded byte: with the bf16 -> fp32
+// unpacking a sweep on the FMA pipe is issue-bound at ~1/8 of the HBM roofline (profiles/: FMA pipe 26 %, 488 M warp
+// instructions for 1.3 GB).  The reduction is a contraction,
 //     out[box][c] += sum_y a_y[box] * ( sum_x b_x[box] * L[y][x][c] ),
 // so the inner sum over a region row runs as mma.sync m16n8k16 (A = b_x of 16 boxes, B = 16 cells x 8 channels of
 // the bf16 map, fp32 accumulate) and only the per-row scaling by a_y stays on the FMA pipe (1 FMA per 32 MACs).
@@ -751,12 +593,11 @@ static size_t image_ws_floats(const fo1_hfre_image& im) {
   for (int l = 0; l < im.n_levels; ++l) f += (size_t)im.n_boxes * level_wstride(im.levels[l]);
   return f;
 }
-static int list_stride(int n_boxes) { return (1 + n_boxes + 3) & ~3; }                 // SIMT sweep: count + ids
-static int record_stride(int n_boxes) { return 4 + n_boxes * kRecWords; }             // tensor sweep: count + 48-word records
+static int record_stride(int n_boxes) { return 4 + n_boxes * kRecWords; }             // count + 48-word records
 static size_t image_list_ints(const fo1_hfre_image& im) {
   size_t n = 0;
   for (int l = 0; l < im.n_levels; ++l)
-    n += (size_t)ceil_div(im.levels[l].H, kMmaRows) * ceil_div(im.levels[l].W, kRegion) * record_stride(im.n_boxes);   // finest region grid / widest list of any algo
+    n += (size_t)ceil_div(im.levels[l].H, kMmaRows) * ceil_div(im.levels[l].W, kRegion) * record_stride(im.n_boxes);
   return n;
 }
 
@@ -782,7 +623,7 @@ extern "C" int fo1_hfre_forward(const fo1_hfre_image* images, int32_t n_images, 
   if (n_images == 0) return FO1_OK;
   FO1_CHECK_ARG(p->roi_size >= 1 && p->roi_size <= 32, "fo1_hfre_forward: roi_size %d unsupported", p->roi_size);
   FO1_CHECK_ARG(p->out_dim > 0 && p->out_dim % 4 == 0, "fo1_hfre_forward: out_dim %d must be a positive multiple of 4", p->out_dim);
-  FO1_CHECK_ARG(p->algo >= 0 && p->algo <= 3, "fo1_hfre_forward: algo %d not available", p->algo);
+  FO1_CHECK_ARG(p->algo == 0 || p->algo == 1 || p->algo == 3, "fo1_hfre_forward: algo %d not available (0 auto, 1 gather, 3 sweep)", p->algo);
   const size_t need = fo1_hfre_workspace_bytes(images, n_images, p);
   if (workspace == nullptr || workspace_bytes < need) {
     set_error("fo1_hfre_forward: workspace %zu B < required %zu B", workspace_bytes, need);
@@ -810,11 +651,8 @@ extern "C" int fo1_hfre_forward(const fo1_hfre_image* images, int32_t n_images, 
     B.pos = p->apply_pos_embed ? 1 : 0;
     int batch_boxes = 0;
     for (int i = 0; i < B.n_images; ++i) batch_boxes += images[base + i].n_boxes > 0 ? images[base + i].n_boxes : 0;
-    // algo 0: a sweep wins as soon as boxes overlap (its traffic is the union of the windows, the gather's their sum),
-    // and the tensor-pipe sweep beats the SIMT one at every density measured (profiles/r01_microbench_hfre_*.json)
-    const bool sweep = p->algo == 2 || p->algo == 3 || (p->algo == 0 && batch_boxes >= 8 * B.n_images);
-    const bool tensor = p->algo == 3 || (p->algo == 0 && sweep);
-    B.rrows = tensor ? kMmaRows : kRegion;
+    // algo 0: the sweep wins as soon as boxes overlap (its traffic is the union of the windows, the gather's their sum)
+    const bool sweep = p->algo == 3 || (p->algo == 0 && batch_boxes >= 8 * B.n_images);
     int max_boxes = 0, max_levels = 0, max_chunks = 0, max_up = 0, max_hw = 0, max_items = 0, max_regions = 0;
     for (int i = 0; i < B.n_images; ++i) {
       const fo1_hfre_image& src = images[base + i];
@@ -836,7 +674,7 @@ extern "C" int fo1_hfre_forward(const fo1_hfre_image* images, int32_t n_images, 
       d.ws_ofs = (long long)ws_ofs;
       int wofs = 0, chunks = 0, lofs = 0, items = 0;
       d.ls_ofs = (long long)ls_ofs;
-      d.lstride = tensor ? record_stride(src.n_boxes) : list_stride(src.n_boxes);
+      d.lstride = record_stride(src.n_boxes);
       for (int l = 0; l < src.n_levels; ++l) {
         const fo1_hfre_level& sl = src.levels[l];
         FO1_CHECK_ARG(sl.data != nullptr && sl.H > 0 && sl.W > 0 && sl.C > 0, "image %d level %d: bad shape", base + i, l);
@@ -854,7 +692,7 @@ extern "C" int fo1_hfre_forward(const fo1_hfre_image* images, int32_t n_images, 
         dl.wstride = level_wstride(sl);
         wofs += src.n_boxes * dl.wstride;
         chunks += ceil_div(sl.C, kChunk);
-        dl.rh = ceil_div(sl.H, B.rrows); dl.rw = ceil_div(sl.W, kRegion);
+        dl.rh = ceil_div(sl.H, kMmaRows); dl.rw = ceil_div(sl.W, kRegion);
         dl.lofs = lofs;
         lofs += dl.rh * dl.rw * d.lstride;
         items += dl.rh * dl.rw * ceil_div(sl.C, kSweepCh);
@@ -891,21 +729,17 @@ extern "C" int fo1_hfre_forward(const fo1_hfre_image* images, int32_t n_images, 
       }
       {
         dim3 grid(max_regions, max_levels, B.n_images);
-        if (tensor) hfre_region_records_kernel<<<grid, 128, 0, stream>>>(B, ws, lists);
-        else hfre_region_lists_kernel<<<grid, 32, 0, stream>>>(B, ws, lists);
+        hfre_region_records_kernel<<<grid, 128, 0, stream>>>(B, ws, lists);
         FO1_LAUNCH_CHECK();
       }
       dim3 grid(max_items, 1, B.n_images);
-      ProfScope prof(tensor ? "hfre_sweep_mma" : "hfre_sweep", 0.0, 0.0, stream);
-      if (tensor) {
-        static bool attr_set = false;
-        if (!attr_set) {
-          FO1_CUDA(cudaFuncSetAttribute(hfre_sweep_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMmaSmemBytes));
-          attr_set = true;
-        }
-        hfre_sweep_mma_kernel<<<grid, kSweepThreads, kMmaSmemBytes, stream>>>(B, ws, lists);
+      ProfScope prof("hfre_sweep_mma", 0.0, 0.0, stream);
+      static bool attr_set = false;
+      if (!attr_set) {
+        FO1_CUDA(cudaFuncSetAttribute(hfre_sweep_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMmaSmemBytes));
+        attr_set = true;
       }
-      else hfre_sweep_kernel<<<grid, kSweepThreads, 0, stream>>>(B, ws, lists);
+      hfre_sweep_mma_kernel<<<grid, kSweepThreads, kMmaSmemBytes, stream>>>(B, ws, lists);
       FO1_LAUNCH_CHECK();
     } else {
       dim3 grid(max_chunks, max_boxes, B.n_images);

@@ -532,11 +532,9 @@ static int llm_generate_impl(Model* m, fo1_generate_desc* d, cudaStream_t s, boo
   int* d_deltas = A.alloc<int>(B);
   // persistent decode kernel (decode_mega.cu): per-CTA slots + the grid barrier
   // measured with warm clocks, alternating the two paths (scripts/mega_prof.py, profiles/README.md round 2): the persistent kernel
-  // beats the per-kernel graph at every batch it supports (1..32 sequences: -8 % .. -19 % per step).  FO1_MEGA_MAX_B lowers the
-  // threshold, FO1_NO_MEGA disables the kernel.
-  int mega_max_b = 32;
-  if (const char* e = getenv("FO1_MEGA_MAX_B")) mega_max_b = std::max(0, std::min(32, atoi(e)));
-  const int mega_grid = (m->llm.mega_ok && B <= mega_max_b && getenv("FO1_NO_MEGA") == nullptr) ? decode_mega_grid() : 0;
+  // beats the per-kernel graph at every batch it supports (1..32 sequences: -8 % .. -19 % per step).  FO1_NO_MEGA disables the
+  // kernel.
+  const int mega_grid = (m->llm.mega_ok && B <= 32 && getenv("FO1_NO_MEGA") == nullptr) ? decode_mega_grid() : 0;
   float* mg_ssq = A.alloc<float>((size_t)2 * std::max(mega_grid, 1) * 32);
   float* mg_amax_v = A.alloc<float>((size_t)std::max(mega_grid, 1) * 32);
   int* mg_amax_i = A.alloc<int>((size_t)std::max(mega_grid, 1) * 32);
@@ -601,9 +599,8 @@ static int llm_generate_impl(Model* m, fo1_generate_desc* d, cudaStream_t s, boo
   // step runs eagerly (warms every kernel), the second is captured into a CUDA graph that is replayed afterwards ----
   LlmState* ls = static_cast<LlmState*>(m->llm_state);
   // programmatic dependent launch: each kernel of the step starts (prologue, weight prefetch) while its predecessor drains
-  const bool use_pdl = getenv("FO1_NO_PDL") == nullptr;
   auto enqueue_step = [&]() -> int {
-    PdlScope pdl(use_pdl);
+    PdlScope pdl(true);
     SplitKScope sk(true);       // M = number of sequences in every GEMM of a decode step
     launch_k(embed_tokens_kernel, dim3(B), dim3(256), 0, s, st.cur_tok, m->llm.embed, xa, H);
     FO1_LAUNCH_CHECK();
@@ -704,7 +701,7 @@ static int llm_generate_impl(Model* m, fo1_generate_desc* d, cudaStream_t s, boo
   }
   cudaGraphExec_t gexec = nullptr;
   m->last_decode_path = 0;
-  const bool want_graph = !g_prof_on && d->max_new_tokens > 3 && getenv("FO1_NO_GRAPH") == nullptr;
+  const bool want_graph = !g_prof_on && d->max_new_tokens > 3;
   d->steps_run = 0;
   int rc = FO1_OK;
   for (int step = 1; step < d->max_new_tokens; ++step) {

@@ -29,7 +29,7 @@ class HfreConfig:
     vt_mode: str = "fpn"                  # 'fpn' (mm_use_simpleFPN_for_vt) | 'concat'
     roi_size: int = 7                     # mm_roi_output_size
     apply_pos_embed: bool = True          # mm_apply_position_embedding (bbox_based)
-    algo: int = 0
+    algo: int = 0                         # fo1_hfre_params.algo: 0 auto, 1 per-box gather, 3 map sweep
 
 
 class HfreWorkspace:
@@ -47,36 +47,51 @@ class HfreWorkspace:
 _default_ws = HfreWorkspace()
 
 
-def _fill_image(img: HfreImage, aux_feats, vt_feats, boxes_aux, boxes_vt, out, out_bf16, cfg, vt_grid_hw):
-    levels = []
-    H0 = max(f.shape[0] for f in aux_feats)
-    W0 = max(f.shape[1] for f in aux_feats)
-    off = 0
-    for f in aux_feats:  # aux levels are up-sampled to level 0's grid by the reference (:338-350)
-        levels.append((f, H0, W0, AUX_SCALE, 0, off))
-        off += f.shape[2]
+def _level_table(aux_shapes, vt_shapes, cfg: HfreConfig):
+    """``(up_H, up_W, spatial_scale, box_set, out_offset)`` of every level, aux levels first, from the levels' native
+    ``(H, W, C)`` shapes."""
+    H0 = max(s[0] for s in aux_shapes)
+    W0 = max(s[1] for s in aux_shapes)
     if cfg.vt_mode == "fpn":
-        for i, f in enumerate(vt_feats):
-            levels.append((f, f.shape[0], f.shape[1], 1.0 / FPN_STRIDES[i], 1, off))
-            off += f.shape[2]
+        vt_scales = [1.0 / FPN_STRIDES[i] for i in range(len(vt_shapes))]
     elif cfg.vt_mode == "concat":
-        for f in vt_feats:
-            levels.append((f, f.shape[0], f.shape[1], VT_SCALE, 1, off))
-            off += f.shape[2]
+        vt_scales = [VT_SCALE] * len(vt_shapes)
     else:
         raise ValueError(f"unknown vt_mode {cfg.vt_mode!r}")
+    rows = []
+    off = 0
+    for s in aux_shapes:  # aux levels are up-sampled to level 0's grid by the reference (:338-350)
+        rows.append((H0, W0, AUX_SCALE, 0, off))
+        off += s[2]
+    for s, sc in zip(vt_shapes, vt_scales):
+        rows.append((s[0], s[1], sc, 1, off))
+        off += s[2]
     if off > cfg.region_dim:
         raise ValueError(f"levels provide {off} channels > region_dim {cfg.region_dim}")
-    if len(levels) > _lib.FO1_HFRE_MAX_LEVELS:
+    if len(rows) > _lib.FO1_HFRE_MAX_LEVELS:
         raise ValueError("too many feature levels")
-    for i, (f, uh, uw, sc, bs, o) in enumerate(levels):
+    return rows
+
+
+def _launch(imgs, n_images: int, cfg: HfreConfig, dev, workspace: Optional[HfreWorkspace]) -> None:
+    p = HfreParams(cfg.region_dim, cfg.roi_size, 1 if cfg.apply_pos_embed else 0, cfg.algo)
+    L = lib()
+    need = L.fo1_hfre_workspace_bytes(imgs, n_images, C.byref(p))
+    ws = (workspace or _default_ws).get(need, dev)
+    check(L.fo1_hfre_forward(imgs, n_images, C.byref(p), C.c_void_p(ws.data_ptr()), ws.numel(),
+                             C.c_void_p(torch.cuda.current_stream().cuda_stream)), "fo1_hfre_forward")
+
+
+def _fill_image(img: HfreImage, aux_feats, vt_feats, boxes_aux, boxes_vt, out, out_bf16, cfg, vt_grid_hw):
+    rows = _level_table([f.shape for f in aux_feats], [f.shape for f in vt_feats], cfg)
+    for i, (f, (uh, uw, sc, bs, o)) in enumerate(zip(list(aux_feats) + list(vt_feats), rows)):
         if f.dtype != torch.bfloat16 or not f.is_contiguous() or f.dim() != 3 or not f.is_cuda:
             raise _lib.Fo1Error("HFRE levels must be contiguous channels-last bf16 CUDA tensors [H, W, C]")
         L = img.levels[i]
         L.data = f.data_ptr(); L.H, L.W, L.C = f.shape
         L.up_H, L.up_W = uh, uw
         L.spatial_scale = sc; L.box_set = bs; L.out_offset = o
-    img.n_levels = len(levels)
+    img.n_levels = len(rows)
     img.n_boxes = boxes_aux.shape[0]
     img.boxes_aux = boxes_aux.data_ptr(); img.boxes_vt = boxes_vt.data_ptr()
     img.out = out.data_ptr()
@@ -107,13 +122,7 @@ def hfre_forward(aux_feats: Sequence[Sequence[torch.Tensor]], vt_feats: Sequence
         o16 = torch.empty((n, cfg.region_dim), dtype=torch.bfloat16, device=ba.device) if want_bf16 else None
         outs.append(o); outs16.append(o16)
         _fill_image(imgs[b], aux_feats[b], vt_feats[b], ba, bv, o, o16, cfg, vt_grid_hw[b])
-    p = HfreParams(cfg.region_dim, cfg.roi_size, 1 if cfg.apply_pos_embed else 0, cfg.algo)
-    L = lib()
-    need = L.fo1_hfre_workspace_bytes(imgs, B, C.byref(p))
-    dev = outs[0].device if outs else torch.device("cuda")
-    ws = (workspace or _default_ws).get(need, dev)
-    check(L.fo1_hfre_forward(imgs, B, C.byref(p), C.c_void_p(ws.data_ptr()), ws.numel(),
-                             C.c_void_p(torch.cuda.current_stream().cuda_stream)), "fo1_hfre_forward")
+    _launch(imgs, B, cfg, outs[0].device if outs else torch.device("cuda"), workspace)
     return (outs, outs16) if want_bf16 else outs
 
 
@@ -137,37 +146,21 @@ def hfre_forward_packed(aux_levels: Sequence[torch.Tensor], vt_levels: Sequence[
     total = int(sum(counts))
     if boxes_aux.shape != (total, 4) or boxes_vt.shape != (total, 4):
         raise _lib.Fo1Error("HFRE packed boxes do not match counts")
-    H0 = max(f.shape[1] for f in aux_levels); W0 = max(f.shape[2] for f in aux_levels)
-    levels = []
-    off = 0
-    for f in aux_levels:
-        levels.append((f, H0, W0, AUX_SCALE, 0, off)); off += f.shape[3]
-    if cfg.vt_mode == "fpn":
-        for i, f in enumerate(vt_levels):
-            levels.append((f, f.shape[1], f.shape[2], 1.0 / FPN_STRIDES[i], 1, off)); off += f.shape[3]
-    elif cfg.vt_mode == "concat":
-        for f in vt_levels:
-            levels.append((f, f.shape[1], f.shape[2], VT_SCALE, 1, off)); off += f.shape[3]
-    else:
-        raise ValueError(f"unknown vt_mode {cfg.vt_mode!r}")
-    if off > cfg.region_dim:
-        raise ValueError(f"levels provide {off} channels > region_dim {cfg.region_dim}")
-    if len(levels) > _lib.FO1_HFRE_MAX_LEVELS:
-        raise ValueError("too many feature levels")
+    rows = _level_table([f.shape[1:] for f in aux_levels], [f.shape[1:] for f in vt_levels], cfg)
     out = torch.empty((total, cfg.region_dim), dtype=torch.float32, device=dev)
     out16 = torch.empty((total, cfg.region_dim), dtype=torch.bfloat16, device=dev) if want_bf16 else None
     imgs = (HfreImage * B)()
     a = np.frombuffer(imgs, dtype=_IMG_DTYPE)
     idx = np.arange(B, dtype=np.uint64)
     lv = a["levels"]
-    for i, (f, uh, uw, sc, bs, o) in enumerate(levels):
+    for i, (f, (uh, uw, sc, bs, o)) in enumerate(zip(list(aux_levels) + list(vt_levels), rows)):
         lv["data"][:, i] = np.uint64(f.data_ptr()) + idx * np.uint64(f.stride(0) * 2)
         lv["H"][:, i], lv["W"][:, i], lv["C"][:, i] = f.shape[1], f.shape[2], f.shape[3]
         lv["up_H"][:, i], lv["up_W"][:, i] = uh, uw
         lv["spatial_scale"][:, i] = sc; lv["box_set"][:, i] = bs; lv["out_offset"][:, i] = o
     cnt = np.asarray(counts, dtype=np.uint64)
     row0 = np.concatenate([[0], np.cumsum(cnt)[:-1]]).astype(np.uint64)
-    a["n_levels"] = len(levels)
+    a["n_levels"] = len(rows)
     a["n_boxes"] = cnt.astype(np.int32)
     a["boxes_aux"] = np.uint64(boxes_aux.data_ptr()) + row0 * np.uint64(16)
     a["boxes_vt"] = np.uint64(boxes_vt.data_ptr()) + row0 * np.uint64(16)
@@ -177,12 +170,7 @@ def hfre_forward_packed(aux_levels: Sequence[torch.Tensor], vt_levels: Sequence[
     a["pos_img_w"] = gw / VT_SCALE      # :447-448 (python float, rounded to fp32 at the division like the reference)
     a["pos_img_h"] = gh / VT_SCALE
     a["pos_box_set"] = 1
-    p = HfreParams(cfg.region_dim, cfg.roi_size, 1 if cfg.apply_pos_embed else 0, cfg.algo)
-    L = lib()
-    need = L.fo1_hfre_workspace_bytes(imgs, B, C.byref(p))
-    ws = (workspace or _default_ws).get(need, dev)
-    check(L.fo1_hfre_forward(imgs, B, C.byref(p), C.c_void_p(ws.data_ptr()), ws.numel(),
-                             C.c_void_p(torch.cuda.current_stream().cuda_stream)), "fo1_hfre_forward")
+    _launch(imgs, B, cfg, dev, workspace)
     return (out, out16) if want_bf16 else out
 
 
